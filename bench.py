@@ -1,14 +1,16 @@
 #!/usr/bin/env python
 """bench.py -- MAC reasoning steps/sec on synthetic CLEVR-shaped batches (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--prec bf16|fp32] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--prec bf16|fp32] [--impl ours|reference] [--dump-outputs DIR]
 
 A bench "step" is one full pass of the hot path over one batch: the netLength-step unroll of the MAC cell
 (model.py:447-458) on B=64 questions -- 12 reasoning steps at the headline configuration (BASELINE.json
 configs[2]: B=64, S=40, 14x14 KB, d=512, netLength=12).  `value` = reasoning steps/s = K * netLength * N / t.
 
   value   inputs resident in HBM when the timed region starts; the K timed passes rotate over 8 resident
-          batches (8 x 31 MB > 126 MB L2) so the knowledge base comes from HBM every pass.
+          batches (8 x 31 MB > 126 MB L2) so the knowledge base comes from HBM every pass.  `--dump-outputs DIR`
+          writes what the last of them returned (final control and memory, both attention maps) as DIR/<name>.npy,
+          float32; inputs and weights are seeded, so two builds run with the same arguments can be compared.
   e2e     the same metric through the public API with HOST (pinned) buffers: per pass the H2D copy of the batch
           (KB, words, question vector, lengths) and the D2H read of the final state + attention maps are inside the
           timed region (double-buffered against compute on a copy stream).
@@ -236,8 +238,15 @@ class Slot(object):
             self._net(self.cell, self.L)
 
     def outputs(self):
+        """What a caller of the pass receives, under the names serving.HostPipeline returns them by."""
         c = self.cell
-        return [c._hc[self.L], c._hm[self.L], c._att_kb, c._att_q]
+        return {"control": c._hc[self.L], "memory": c._hm[self.L], "att_kb": c._att_kb, "att_question": c._att_q}
+
+
+def dump_outputs(outdir, outputs):
+    os.makedirs(outdir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(outdir, name + ".npy"), t.float().cpu().numpy())
 
 
 def ncu_traffic(key):
@@ -599,11 +608,14 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    # K = --steps passes per block, blocks repeated until >= 0.5 s of device time: the reported time is the MEDIAN block
+    # K = --steps passes per block, blocks repeated until >= --min-time s of device time (default: one block): the reported
+    # time is the MEDIAN block
     t_dev, dev_blocks = timed_blocks(run_passes, args.steps, barrier, dist, min_total_s=args.min_time)
     # the sampler stops HERE: polling nvidia-smi through the host-driven end-to-end region below costs it ~15 % (19.8k vs
     # 23.5k reasoning-steps/s on the B200 box, profiles/r1/NOTES.md) -- the queries contend with the copy / launch calls
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:       # every block runs passes 0..K-1, so pass K-1 used slot (K-1) % nslots last
+        dump_outputs(args.dump_outputs, slots[(args.steps - 1) % nslots].outputs())
 
     # ---- end-to-end arm: host (pinned) buffers; every pass does H2D of its batch, the netLength unroll, and D2H of the
     #      final state + attention maps.  ND device slots, each on its own stream, so the copies of one pass overlap the
@@ -686,7 +698,8 @@ def run_ours(args):
             "config": {"workload": workload_string(shape),
                        "step": "one netLength-step unroll over one batch (%d reasoning steps)" % L,
                        "timing": "blocks of exactly --steps passes (barrier + synchronize on both sides, CUDA events, max over "
-                                 "ranks), repeated until >= %.2f s; ms_per_step / value are the MEDIAN block" % args.min_time,
+                                 "ranks), repeated until >= %.2f s (0: one block); ms_per_step / value are the MEDIAN block"
+                                 % args.min_time,
                        "l2": "timed passes rotate over %d resident batches (%.0f MB > 126 MB L2)"
                              % (nslots, nslots * (B * N * d + B * S * d) * 4 / 1e6),
                        "cuda_graph": use_graph, "projections": args.prec, "concurrent_passes": nstreams,
@@ -974,10 +987,11 @@ def run_quick(args):
 
 
 def child_measure(extra, timeout_s=60):
-    """Run `bench.py <extra>` in a child process and return its last JSON line (or an error record)."""
+    """Run `bench.py <extra>` in a child process and return its last JSON line (or an error record).  The side
+    measurements take few passes, so their block is repeated until 0.5 s is timed."""
     try:
-        out = subprocess.run([sys.executable, os.path.abspath(__file__)] + extra, capture_output=True, text=True,
-                             timeout=timeout_s, cwd=ROOT)
+        out = subprocess.run([sys.executable, os.path.abspath(__file__), "--min-time", "0.5"] + extra, capture_output=True,
+                             text=True, timeout=timeout_s, cwd=ROOT)
         if out.returncode != 0:
             return {"error": "exit %d: %s" % (out.returncode, out.stderr.strip()[-300:])}
         return json.loads(out.stdout.strip().splitlines()[-1])
@@ -1038,11 +1052,18 @@ def main():
                     "measured on the B200 (packed read step): 1: 19.9k, 4: 32.4k, 8: 34.4k, 12: 35.1k, 16: 35.1k reasoning-steps/s")
     ap.add_argument("--fold-y", type=int, default=-1, help="write unit folded with the next step's projY: 1/0, -1 = by --streams")
     ap.add_argument("--rooflines-only", action="store_true", help="only the per-kernel measurements (for ncu)")
-    ap.add_argument("--min-time", type=float, default=0.5, help="repeat the --steps block until this many seconds are timed")
+    ap.add_argument("--min-time", type=float, default=0.0, help="repeat the --steps block until this many seconds are timed "
+                    "(default: one block, so exactly --steps passes are timed)")
     ap.add_argument("--workload", default="headline", choices=["headline", "gqa", "cpu_ref"], help="--mode quick: shape + flag file")
     ap.add_argument("--train-prec", default="fp32", choices=["fp32", "bf16"], help="--mode train: read-unit forward GEMMs")
     ap.add_argument("--bwd-tc", type=int, default=0, help="--mode train: read-unit backward GEMMs on tensor cores (1/0)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed pass of the resident-input arm returned "
+                    "(rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.rooflines_only or args.impl != "ours" or args.mode != "infer"):
+        ap.error("--dump-outputs applies to the default inference run only")
     args.warmup = max(args.warmup, 3)
     if args.rooflines_only:
         torch.cuda.set_device(0)

@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = ["metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
              "vs_baseline", "dtype", "data", "config"]
@@ -57,3 +60,28 @@ def test_reference_arm_line_live():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0
     assert line["e2e"]["value"] == line["value"] == line["cpu_baseline"]["value"]
     assert line["cpu_baseline"]["cores"] >= 1
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_from_run_to_run(tmp_path):
+    """`--steps K` times exactly K passes (one block), and `--dump-outputs` writes what the last of them returned: two runs
+    with the same arguments write the same arrays."""
+    from mac_network_b200.synthetic import SHAPES
+    B, S, N, d, L = SHAPES["headline"]
+    shapes = {"control": (B, d), "memory": (B, d), "att_kb": (L, B, N), "att_question": (L, B, S)}
+    dumps = []
+    for run in range(2):
+        out_dir = str(tmp_path / ("run%d" % run))
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "3", "--skip-train",
+                              "--skip-cpu", "--dump-outputs", out_dir], capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-800:]
+        line = json.loads(out.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 3 and line["timed_blocks"]["resident"]["blocks"] == 1
+        assert sorted(os.listdir(out_dir)) == sorted(k + ".npy" for k in shapes)
+        dumps.append({k: np.load(os.path.join(out_dir, k + ".npy")) for k in shapes})
+    for k, shape in shapes.items():
+        assert dumps[0][k].dtype == np.float32 and dumps[0][k].shape == shape, k
+        assert np.isfinite(dumps[0][k]).all(), k
+        assert np.array_equal(dumps[0][k], dumps[1][k]), k
+    for k in ("att_kb", "att_question"):
+        assert np.allclose(dumps[0][k].sum(-1), 1.0, atol=1e-5), k

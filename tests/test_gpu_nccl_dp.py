@@ -2,7 +2,7 @@
 hand-written forward/backward kernels on its half of the batch and all-reducing the flat gradient bucket over NCCL, must
 reproduce the gradient one process computes on the concatenated batch (eval-mode dropouts, so the shards see the same
 function), and after the fused clip/Adam/EMA step the replicas must hold bit-identical weights.
-Needs 2 GPUs (skipped on the 1-GPU box the driver uses; run with `gpurun --gpus 2`)."""
+Needs 2 GPUs (skipped on a machine with one)."""
 import os
 import sys
 
@@ -52,7 +52,7 @@ def _worker(rank, world, port, out_dir):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_two_rank_nccl_cuda_gradient_equals_single_process(tmp_path):
     import torch.multiprocessing as mp
     from mac_network_b200.dp import DPTrainer
